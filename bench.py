@@ -25,6 +25,10 @@ One JSON line (rank 0):
 
 `--impl reference` times that CPU restatement alone (the Python reference itself cannot travel to the GPU box).
 
+`--dump-outputs DIR` writes, after the run, the latents x_{t-1} that the last timed step returned, as
+DIR/latents.npy (float32, [16, 4, 64, 64]; DIR/latents_rank<k>.npy per rank when N > 1).  Weights and inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
+
 Multi-GPU (`--gpus N` under torchrun): local merging makes frame chunks independent (generate.py:216-219), so
 each rank denoises its own 16-frame chunk with replicated weights; nothing crosses GPUs in the data path
 ("scaling": "weak").  Timing = max over ranks of the CUDA-event time between two barriers.
@@ -468,6 +472,7 @@ def run_ours(args):
         dev_step(i)
     sampler = ClockSampler(local, str(getattr(torch.cuda.get_device_properties(local), "uuid", "") or "")) if rank == 0 else None
     ms = timed(dev_step, args.steps)
+    last_x = state["x"]                                        # what the last timed step returned
     if sampler and world == 1 and sampler.mode is not None:
         # a timed region shorter than the sampler's period: keep the SAME workload running (untimed) until it has
         # a few samples under load, and say so
@@ -596,6 +601,11 @@ def run_ours(args):
         wd.cancel()
         if rank == 0:
             line["c4_global"] = c4
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "latents" if world == 1 else f"latents_rank{rank}"
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), last_x.float().cpu().numpy())
     emit()
     if world > 1:
         dist.destroy_process_group()
@@ -640,7 +650,11 @@ def main():
     ap.add_argument("--no-c4-global", action="store_true",
                     help="N > 1: skip the secondary BASELINE config-4 block (global-token exchange: all-gather and fused p2p)")
     ap.add_argument("--c4-timeout", type=int, default=240, help="watchdog for the config-4 block, seconds")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latents returned by the last timed step to DIR/latents.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times block calls, not steps)")
     _claim_stdout()
     if args.impl == "reference":
         run_reference(args)

@@ -1,50 +1,37 @@
 """The torch-op comparator that bench.py times beside the CUDA path (baseline/torch_reference_path.py) must BE the
-reference's formulation: where the reference tree is available (the build container), its patched block and the
-restatement produce identical outputs on the same skeleton with the same random draws.  Skipped on the GPU box."""
+reference's formulation: on the same skeleton with the same random draws it reproduces, bit for bit, the output of the
+reference's own patched UNet, stored in tests/golden/restatement_tiny_f*.npz by `tests/make_golden_r02.py --restatement`."""
 import os
 import sys
 
+import numpy as np
 import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "vidtome")), reason="reference tree not present")
 @pytest.mark.parametrize("frames", [4, 8])
 def test_restatement_equals_reference_on_cpu(frames, monkeypatch):
     sys.path.insert(0, ROOT)
     from baseline import torch_reference_path as R
     from vidtome_b200.skeleton import make_skeleton
-    sys.dont_write_bytecode = True
-    sys.path.insert(0, REF)
-    import vidtome as ref
-    real_randint = torch.randint
-    draws = iter([1, 0, 3, 1, 2, 0, 1, 1] * 8)
+    g = np.load(os.path.join(ROOT, "tests", "golden", f"restatement_tiny_f{frames}.npz"))
+    draws = iter(g["draws"].tolist())
 
     def fixed(lo, hi, size, **kw):
         v = next(draws) % hi
         return torch.full(tuple(size), v, dtype=torch.int64)
-    torch.manual_seed(0)
-    x = torch.randn(2 * frames, 4, 16, 16)
-    outs = []
-    for which in ("reference", "restatement"):
-        net = make_skeleton("tiny", device="cpu", dtype=torch.float32, hot_path_only=False, seed=5)
-        draws = iter([1, 0, 3, 1, 2, 0, 1, 1] * 8)
-        monkeypatch.setattr(torch, "randint", fixed)
-        # the reference's CPU argsort is not stable; force the (CUDA-like) stable order on both sides
-        real_argsort = torch.Tensor.argsort
-        monkeypatch.setattr(torch.Tensor, "argsort", lambda t, *a, **k: real_argsort(t, *a, **{**k, "stable": True}))
-        if which == "reference":
-            ref.apply_patch(net, local_merge_ratio=0.9, batch_size=2)
-        else:
-            R.apply_reference_path(net, 0.9, 2)
-        with torch.no_grad():
-            outs.append(net(x, 0, encoder_hidden_states=torch.zeros(2 * frames, 7, 768)).sample)
-        monkeypatch.setattr(torch, "randint", real_randint)
-        monkeypatch.setattr(torch.Tensor, "argsort", real_argsort)
-    assert torch.equal(outs[0], outs[1])
+    x = torch.from_numpy(g["x"])
+    net = make_skeleton("tiny", device="cpu", dtype=torch.float32, hot_path_only=False, seed=5)
+    monkeypatch.setattr(torch, "randint", fixed)
+    # the reference's CPU argsort is not stable; the fixture was made with the (CUDA-like) stable order
+    real_argsort = torch.Tensor.argsort
+    monkeypatch.setattr(torch.Tensor, "argsort", lambda t, *a, **k: real_argsort(t, *a, **{**k, "stable": True}))
+    R.apply_reference_path(net, 0.9, 2)
+    with torch.no_grad():
+        out = net(x, 0, encoder_hidden_states=torch.zeros(2 * frames, 7, 768)).sample
+    assert torch.equal(out, torch.from_numpy(g["out"]))
 
 
 def test_config1_plumbing_on_cpu():
