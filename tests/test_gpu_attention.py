@@ -40,7 +40,7 @@ def test_attention_matches_fp32_reference(B, L, C, heads):
     ref = _ref_attention(x, ws[0], ws[1], ws[2], ws[3], bo, heads, scale)
     err = (y.float() - ref).abs().max().item()
     assert torch.isfinite(y).all()
-    assert err <= 1e-3 * ref.abs().max().item() + 2e-3, err      # 1e-3 relative fp16 tolerance (+ fp16 rounding of y)
+    assert err <= 1e-3 * ref.abs().max().item(), err      # measured on a B200: at most 4.9e-4 x max|ref| over these shapes
 
 
 def test_attention_matches_oracle_small():
@@ -55,7 +55,7 @@ def test_attention_matches_oracle_small():
     y = ops.attention(t(x), torch.cat([t(w[0]), t(w[1]), t(w[2])], 0).contiguous(), t(w[3]), t(bo), heads,
                       (C // heads) ** -0.5)
     err = np.abs(y.float().cpu().numpy() - want).max()
-    assert err <= 1e-3 * np.abs(want).max() + 2e-3, err
+    assert err <= 1.5e-3 * np.abs(want).max(), err      # measured on a B200: 4.9e-4 (one fp16 ulp) = 5.7e-4 x max|want|
 
 
 def test_attention_full_size_c2_ds1_vs_sdpa():
@@ -72,7 +72,7 @@ def test_attention_full_size_c2_ds1_vs_sdpa():
     o = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2).reshape(B, L, C)
     ref = (o @ ws[3].t()).float()
     err = (y.float() - ref).abs().max().item()
-    assert err <= 2e-3 * ref.abs().max().item() + 2e-3, err
+    assert err <= 2e-3 * ref.abs().max().item(), err      # measured on a B200: 2.4e-4 (one fp16 ulp) = 7.2e-4 x max|ref|
 
 
 def test_patched_block_uses_cuda_attention(monkeypatch):
@@ -174,9 +174,10 @@ def test_cross_attention_matches_fp32_reference(B, Lq, Lk, C, Cctx, heads):
     o = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2).reshape(B, Lq, C)
     ref = o @ wo.float().t() + bo.float() + resid.float()
     err = (y.float() - ref).abs().max().item()
-    assert err <= 1e-3 * ref.abs().max().item() + 2e-3
+    assert err <= 1e-3 * ref.abs().max().item()      # measured on a B200: at most 4.4e-4 x max|ref| over these shapes
     y2 = ops.cross_attention(x, ctx, wq, torch.cat([wk, wv], 0).contiguous(), wo, bo, heads, d ** -0.5)
-    assert (y2.float() - (ref - resid.float())).abs().max().item() <= 1e-3 * ref.abs().max().item() + 2e-3
+    # measured on a B200: at most 2.6e-4 x max|ref|
+    assert (y2.float() - (ref - resid.float())).abs().max().item() <= 1e-3 * ref.abs().max().item()
 
 
 def test_full_block_fast_paths_match_module_paths():
@@ -208,7 +209,7 @@ def test_full_block_fast_paths_match_module_paths():
 def test_opt_in_flash_kernels_match_fp32_reference(env):
     """The alternative flash kernels kept for A/B runs (eight softmax warps per CTA, the grouped kernel, the
     non-embedded softmax) are selected by environment variables read once per process: each runs in a child process on
-    shapes that reach the steady-state loop, a masked last tile and the key-range split, at the same 1e-3 tolerance."""
+    shapes that reach the steady-state loop, a masked last tile and the key-range split."""
     import os
     import subprocess
     import sys
@@ -226,7 +227,8 @@ for (B, L, C, H) in [(2, 1000, 320, 8), (3, 1500, 320, 8), (1, 128, 320, 8)]:
     o = ((q @ k.transpose(-1, -2)) * d ** -0.5).softmax(-1) @ v
     ref = o.transpose(1, 2).reshape(B, L, C).half().float() @ ws[3].float().t()
     err = (y.float() - ref).abs().max().item()
-    assert torch.isfinite(y).all() and err <= 1e-3 * ref.abs().max().item() + 2e-3, (L, err)
+    # measured on a B200: at most 7.4e-4 x max|ref| (about one fp16 ulp of y) over the three kernels and shapes
+    assert torch.isfinite(y).all() and err <= 1.5e-3 * ref.abs().max().item(), (L, err)
 print("ok")
 ''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, **env), capture_output=True, text=True, timeout=300)

@@ -47,10 +47,10 @@ def assert_match_tie_aware(level, s_oracle: np.ndarray, om: "O.Match", align: bo
     #     maximum we report is within one ulp of it too
     assert (best - at_ours).max() <= 1, "an arg-max that is not a last-bit tie"
     assert np.abs(_ordered16(nmax) - best).max() <= 1
-    # ... and where the indices differ the oracle sees (near-)equal scores there, with ours never AFTER an exact tie
+    # ... and where the indices differ the oracle sees (near-)equal scores there.  Which index wins an exact tie is not
+    # checked here: the oracle picks the first of its own exact ties, so any comparison with it would hold by construction.
+    # The first-index rule is pinned by the exact-family tests in test_gpu_kernels.py.
     diff = nidx != om.node_idx
-    exact_tie = diff & (at_ours == best)
-    assert (nidx[exact_tie] >= om.node_idx[exact_tie]).all() or True   # first-index rule is checked on exact data
     # (2) order: our edge is exactly the stable descending order of OUR maxima
     edge = level.edge.cpu().numpy()
     want_edge = O.stable_argsort_desc(nmax)

@@ -67,10 +67,10 @@ struct HeadSplitEpi {
     row0 = m_tile * gemm::BM + (row_in_tile & ~31);
     bw = row0 / L;
     lw = row0 - bw * L;
-    // this lane's first row in the store phase: row0 + lane / 8
+    // this lane's first row in the store phase: row0 + lane / 8 (up to 3 rows further: several samples when L < 4)
     b0 = bw;
     l0 = lw + ((row_in_tile & 31) >> 3);
-    if (l0 >= L) { l0 -= L; ++b0; }
+    while (l0 >= L) { l0 -= L; ++b0; }
   }
   // exact x / y for 0 <= x < 2^22 (x + 0.5 keeps the product away from the integer boundary)
   static __device__ __forceinline__ int div_small(int x, float inv_y) {
